@@ -73,6 +73,27 @@ def algorithmic_flops_per_image(unet=UNET, image=IMAGE):
     return fl
 
 
+DUMP_BYTES = 64 << 20                            # all arrays of one --dump-outputs together
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: every array as <out_dir>/<name>.npy (float32, or float64 where computed so).  DUMP_BYTES is split evenly between the
+    arrays; one over its share is replaced by a fixed sample of its flattened elements (the same sorted indices every run, numpy seed 0), so
+    two builds stay comparable."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // max(len(arrays), 1)
+    total = 0
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        a = np.ascontiguousarray(a, dtype=np.float64 if a.dtype == np.float64 else np.float32)
+        if a.nbytes > share:
+            a = a.reshape(-1)[np.unique(np.random.default_rng(0).integers(0, a.size, share // a.itemsize))]
+        total += a.nbytes
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    assert total <= DUMP_BYTES, total
+
+
 def measured_peaks():
     p = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(p):
@@ -219,7 +240,7 @@ def run_reference(args, rank, world):
     warm = min(max(args.warmup, 1), 2)
     cb = cpu_baseline_block(steps, warm)
     v = cb["value"]
-    line = {"impl": "reference", "metric": METRIC, "value": v, "unit": "steps/s", "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
+    line = {"impl": "reference", "metric": METRIC, "value": v, "unit": "steps/s", "n_gpus": args.gpus, "steps": steps, "warmup": warm,
             "ms_per_step": cb["ms_per_step"], "higher_is_better": True, "scaling": args.scaling, "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": {"workload": "sr_sr3_16_128.json sampling, global batch 16, p_sample on host cores", "global_batch": GLOBAL_BATCH,
                        "timed_steps": steps, "timed_warmup": warm},
@@ -307,14 +328,17 @@ def secondary_workloads(dev, peaks, steps=10):
     return out
 
 
-def time_training(dev, per_batch, global_batch, K, W, barrier, dist_mod=None, host_inputs=False):
+def time_training(dev, per_batch, global_batch, K, W, barrier, dist_mod=None, host_inputs=False, dumps=None):
     """K optimizer iterations (model/model.py:48-58: forward in train() mode incl. Dropout -> backward -> Adam, gradient all-reduce overlapped
     with the backward when world > 1) of sr_sr3_16_128.json on this rank's slice of the global batch.  CUDA events, max over ranks.
-    host_inputs: HR / SR come from pinned host memory every step and the loss value is read back (the end-to-end form)."""
+    host_inputs: HR / SR come from pinned host memory every step and the loss value is read back (the end-to-end form).
+    dumps: a dict that receives the loss of the last timed iteration and the parameters it left (all of them, flattened in order)."""
+    import numpy as np
     import torch
     import sr3_b200
     from sr3_b200 import parallel
     torch.manual_seed(0)
+    np.random.seed(0)                                   # the (t, gamma) draw of every iteration: same inputs on every run
     opt = make_opt(SCHED)
     opt["phase"] = "train"                              # orthogonal init (networks.py:110-112)
     net = sr3_b200.define_G(opt).to(dev)
@@ -353,6 +377,9 @@ def time_training(dev, per_batch, global_batch, K, W, barrier, dist_mod=None, ho
     n_buckets = len(tr.buckets.slices)
     import math
     assert all(math.isfinite(l) for l in losses), "training loss is not finite"
+    if dumps is not None:
+        dumps["train_loss"] = np.array([losses[-1]], dtype=np.float64)
+        dumps["train_params"] = torch.cat([p.detach().reshape(-1) for p in net.parameters()]).cpu().numpy()
     del tr, net
     torch.cuda.empty_cache()
     return float(t_ms.item()) / K, comm_ms, losses, n_blocks, n_buckets
@@ -426,10 +453,11 @@ def cpu_train_baseline(steps=2, sample_batch=2, global_batch=64):
 def run_reference_train(args, rank, world):
     if rank != 0:
         return
-    cb = cpu_train_baseline(steps=min(max(args.steps, 1), 3), global_batch=args.train_batch)
+    steps = min(max(args.steps, 1), 3)         # each CPU iteration is seconds, as above
+    cb = cpu_train_baseline(steps=steps, global_batch=args.train_batch)
     v = cb["value"]
     line = {"impl": "reference", "metric": "training steps/sec (sr_sr3_16_128 fwd+bwd+Adam, global batch %d)" % args.train_batch, "value": v, "unit": "steps/s",
-            "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 / v, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
+            "n_gpus": args.gpus, "steps": steps, "warmup": 1, "ms_per_step": 1e3 / v, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
             "dtype": "f32", "data": "synthetic", "config": {"workload": "sr_sr3_16_128.json training step on host cores (bounded sample, see cpu_baseline.sample)",
                                                              "global_batch": args.train_batch},
             "cpu_baseline": {k: cb[k] for k in ("value", "unit", "cores", "kind", "sample", "host_cores")},
@@ -462,8 +490,11 @@ def run_train(args, rank, local, world):
         torch.cuda.synchronize()
 
     dd = dist if world > 1 else None
+    dumps = {} if args.dump_outputs and rank == 0 else None
     with ClockSampler(local) as clk:
-        ms, comm_ms, losses, n_blocks, n_buckets = time_training(dev, per, GB, K, W, barrier, dd, host_inputs=False)
+        ms, comm_ms, losses, n_blocks, n_buckets = time_training(dev, per, GB, K, W, barrier, dd, host_inputs=False, dumps=dumps)
+    if dumps is not None:
+        dump_outputs(args.dump_outputs, dumps)
     e2e_ms, _, _, _, _ = time_training(dev, per, GB, max(3, K // 2), 3, barrier, dd, host_inputs=True)
     cpu = None
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
@@ -499,7 +530,8 @@ def run_train(args, rank, local, world):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=int, default=50,
+                    help="timed steps; --impl reference times at most 8 sampling steps (3 training iterations) and reports the number it timed")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
@@ -511,6 +543,8 @@ def main():
     ap.add_argument("--workload", default="sample", choices=["sample", "train"],
                     help="sample (default): the BASELINE metric; train: configs[3], the training step (fwd + bwd + Adam) at global batch --train-batch")
     ap.add_argument("--train-batch", type=int, default=64)
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the timed path computed in its last step as DIR/<name>.npy (same arguments, same inputs)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -572,6 +606,15 @@ def main():
     with ClockSampler(local) as clk:
         ms = time_resident(eng, cond_h.to(dev), xT_h.to(dev), lo, K, W, T, barrier, dd, dev)
     value = units * K / (ms * 1e-3)
+    dumps = {}
+    if args.dump_outputs:
+        # the images after the last timed step, read before the e2e calls below reuse the engine; all ranks' shards in batch order
+        state = eng.read_state()
+        if world > 1:
+            parts = [torch.empty_like(state) for _ in range(world)]
+            dist.all_gather(parts, state)
+            state = torch.cat(parts)
+        dumps["sample_state"] = state.cpu().numpy()
     step_prof = eng.step_kernel_profile() if eng.uses_step_kernel() else None      # per-op device times of the last timed launch
 
     # the other scaling mode at N > 1, as a supplementary number (same timing rules)
@@ -608,6 +651,9 @@ def main():
     e2e_val = units * K / float(e2e_t.item())
     img_bytes = per * 3 * IMAGE * IMAGE * 4
     net.set_new_noise_schedule(SCHED, dev)
+    if args.dump_outputs and rank == 0:
+        dumps["super_resolution"] = out_h.numpy()     # the finished images the last e2e call returned
+        dump_outputs(args.dump_outputs, dumps)
 
     if rank != 0:
         if world > 1:

@@ -21,6 +21,14 @@ DST = os.path.join(HERE, "_ref")
 PARTS = ("model", "core", "config")
 
 
+def _make_writable(path):
+    for root, _dirs, names in os.walk(path):
+        os.chmod(root, os.stat(root).st_mode | 0o700)
+        for n in names:
+            p = os.path.join(root, n)
+            os.chmod(p, os.stat(p).st_mode | 0o600)
+
+
 def build(verbose=True):
     if not os.path.isdir(os.path.join(SRC, "model")):
         if verbose:
@@ -32,8 +40,10 @@ def build(verbose=True):
         if not os.path.isdir(s):
             continue
         if os.path.isdir(d):
+            _make_writable(d)
             shutil.rmtree(d)
         shutil.copytree(s, d, ignore=shutil.ignore_patterns("__pycache__", "*.pyc"))
+        _make_writable(d)                      # a read-only source keeps its modes in the copy; the next build must be able to replace it
         for root, _dirs, names in os.walk(d):
             for n in sorted(names):
                 p = os.path.join(root, n)

@@ -29,9 +29,8 @@ def pytest_collection_modifyitems(config, items):
 
 @pytest.fixture(scope="session")
 def golden():
-    import torch
-    p = os.path.join(ROOT, "tests", "golden", "sr3_golden.pt")
-    return torch.load(p, map_location="cpu", weights_only=False)
+    import _golden
+    return _golden.load(os.path.join(ROOT, "tests", "golden", "sr3_golden.pt"))
 
 
 @pytest.fixture(scope="session")

@@ -17,11 +17,13 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, REF)
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.dirname(HERE))
 
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 import model.networks as ref_networks  # noqa: E402  (the reference)
+import _golden  # noqa: E402  (tests/_golden.py: the compact storage form)
 from oracle import sr3_oracle as orc  # noqa: E402
 
 torch.set_num_threads(os.cpu_count())
@@ -40,6 +42,11 @@ TINY = dict(in_channel=6, out_channel=3, inner_channel=64, channel_multiplier=[1
 FULL = dict(in_channel=6, out_channel=3, inner_channel=64, channel_multiplier=[1, 2, 4, 8, 8], attn_res=[16], res_blocks=2, dropout=0.2)
 UNCOND = dict(in_channel=3, out_channel=3, inner_channel=64, channel_multiplier=[1, 2, 4, 8, 8], attn_res=[16], res_blocks=2, dropout=0.2)
 BIG = dict(in_channel=6, out_channel=3, inner_channel=64, norm_groups=16, channel_multiplier=[1, 2, 4, 8, 16], attn_res=[], res_blocks=1, dropout=0)
+
+
+def f16(t):
+    """Random inputs are drawn in fp32 and rounded to fp16 values before use, so the file can store them as fp16 without loss."""
+    return t.half().float()
 
 
 def build_ref(unet, image_size, seed, conditional=True, phase="val", sched=SCHED_SR3):
@@ -88,7 +95,7 @@ def main():
 
     # ---- 3. tiny UNet: eps + per-layer taps ----------------------------------------------
     torch.manual_seed(100)
-    x = torch.randn(2, 6, 32, 32)
+    x = f16(torch.randn(2, 6, 32, 32))
     nlv = torch.tensor([[0.7], [0.05]])
     taps = {}
     hooks = []
@@ -103,22 +110,22 @@ def main():
     with torch.no_grad():
         oeps = orc.unet_forward(sd, cfg, x, nlv, otaps)
     print("tiny eps oracle-vs-ref max abs", (oeps - eps).abs().max().item())
-    out["tiny_unet"] = {"seed": 0, "x": x, "noise_level": nlv, "eps": eps, "taps": taps}
+    out["tiny_unet"] = {"seed": 0, "x": x.half(), "noise_level": nlv, "eps": eps, "taps": {k: _golden.sample(v) for k, v in taps.items()}}
 
     # tiny: p_mean_variance, seeded loop, p_losses
     sched10 = {"schedule": "linear", "n_timestep": 10, "linear_start": 1e-6, "linear_end": 1e-2}
     g.set_new_noise_schedule(sched10, "cpu")
     torch.manual_seed(101)
-    cond = torch.rand(2, 3, 32, 32) * 2 - 1
-    xt = torch.randn(2, 3, 32, 32)
+    cond = f16(torch.rand(2, 3, 32, 32) * 2 - 1)
+    xt = f16(torch.randn(2, 3, 32, 32))
     pmv = {}
     with torch.no_grad():
         for t in (9, 5, 1, 0):
             m, lv = g.p_mean_variance(xt, t, True, condition_x=cond)
             pmv[t] = (m.clone(), lv.clone())
     torch.manual_seed(4321)
-    x_T = torch.randn(2, 3, 32, 32)
-    noises = [torch.randn(2, 3, 32, 32) for _ in range(10)]      # noises[i] used at step i
+    x_T = f16(torch.randn(2, 3, 32, 32))
+    noises = [f16(torch.randn(2, 3, 32, 32)) for _ in range(10)]      # noises[i] used at step i
     # replay the same draws inside the reference: randn(shape) then randn_like per step t>0
     draws = [x_T] + [noises[i] for i in reversed(range(1, 10))]
     it = iter(draws)
@@ -130,12 +137,13 @@ def main():
             loop = g.super_resolution(cond, continous=True)
     finally:
         torch.randn, torch.randn_like = orig_randn, orig_randn_like
-    out["tiny_diffusion"] = {"sched": sched10, "cond": cond, "x_t": xt, "pmv": pmv, "x_T": x_T,
-                             "noises": torch.stack(noises), "loop_continous": loop}
+    cond16 = cond.half()                                          # one fp16 copy per input, shared by every entry that uses it
+    out["tiny_diffusion"] = {"sched": sched10, "cond": cond16, "x_t": xt.half(), "pmv": pmv, "x_T": x_T.half(),
+                             "noises": torch.stack(noises).half(), "loop_continous": _golden.sample(loop), "loop_last": loop[-1].clone()}
     # p_losses with the numpy draws replayed and noise injected
     np.random.seed(7)
-    hr = torch.rand(2, 3, 32, 32) * 2 - 1
-    noise = torch.randn(2, 3, 32, 32)
+    hr = f16(torch.rand(2, 3, 32, 32) * 2 - 1)
+    noise = f16(torch.randn(2, 3, 32, 32))
     with torch.no_grad():
         loss = g.p_losses({"HR": hr, "SR": cond}, noise=noise)
     rng = np.random.RandomState(7)
@@ -144,7 +152,7 @@ def main():
     with torch.no_grad():
         oloss = orc.p_losses(sd, cfg, sch10, hr, cond, gamma, noise)
     print("p_losses ref", loss.item(), "oracle", oloss.item())
-    out["tiny_losses"] = {"np_seed": 7, "hr": hr, "sr": cond, "noise": noise, "t": t_draw, "gamma": gamma, "loss": loss.clone()}
+    out["tiny_losses"] = {"np_seed": 7, "hr": hr.half(), "sr": cond16, "noise": noise.half(), "t": t_draw, "gamma": gamma, "loss": loss.clone()}
 
     # ---- 4. full 16->128 config, B=1 ----------------------------------------------------
     g = build_ref(FULL, 128, 0)
@@ -152,23 +160,24 @@ def main():
     nparams = sum(v.numel() for v in sdF.values())
     assert nparams == 97807491, nparams
     torch.manual_seed(200)
-    cond = torch.rand(1, 3, 128, 128) * 2 - 1
-    xt = torch.randn(1, 3, 128, 128)
-    full = {"cond": cond, "x_t": xt, "eps": {}, "pmv": {}}
+    cond = f16(torch.rand(1, 3, 128, 128) * 2 - 1)
+    xt = f16(torch.randn(1, 3, 128, 128))
+    cond16, xt16 = cond.half(), xt.half()
+    full = {"cond": cond16, "x_t": xt16, "eps": {}, "pmv": {}}
     with torch.no_grad():
         for t in (1999, 1000, 1):
             nl = torch.FloatTensor([g.sqrt_alphas_cumprod_prev[t + 1]]).repeat(1, 1)
-            full["eps"][t] = g.denoise_fn(torch.cat([cond, xt], 1), nl).clone()
+            full["eps"][t] = _golden.sample(g.denoise_fn(torch.cat([cond, xt], 1), nl))
             m, lv = g.p_mean_variance(xt, t, True, condition_x=cond)
-            full["pmv"][t] = (m.clone(), lv.clone())
+            full["pmv"][t] = (_golden.sample(m), lv.clone())
     out["full_16_128"] = full
     # orthogonal (train-phase) init, one eps
     g = build_ref(FULL, 128, 3, phase="train")
     check_init(g, FULL, 128, 3, orthogonal=True)
     with torch.no_grad():
         nl = torch.FloatTensor([[0.285262383882]])
-        out["full_16_128_orth"] = {"seed": 3, "cond": cond, "x_t": xt, "noise_level": nl,
-                                   "eps": g.denoise_fn(torch.cat([cond, xt], 1), nl).clone()}
+        out["full_16_128_orth"] = {"seed": 3, "cond": cond16, "x_t": xt16, "noise_level": nl,
+                                   "eps": _golden.sample(g.denoise_fn(torch.cat([cond, xt], 1), nl))}
 
     # ---- 5. unconditional + 64->512: param counts and a cropped eps -------------------------
     g = build_ref(UNCOND, 128, 0, conditional=False)
@@ -176,7 +185,7 @@ def main():
     assert sum(v.numel() for v in sdU.values()) == 97805763
     with torch.no_grad():
         nl = torch.FloatTensor([[0.5]])
-        out["uncond_128"] = {"x_t": xt, "noise_level": nl, "eps": g.denoise_fn(xt, nl).clone()}
+        out["uncond_128"] = {"x_t": xt16, "noise_level": nl, "eps": _golden.sample(g.denoise_fn(xt, nl))}
     g = build_ref(BIG, 512, 0)
     cfgB, sdB = check_init(g, BIG, 512, 0)
     assert sum(v.numel() for v in sdB.values()) == 155334339
@@ -185,11 +194,13 @@ def main():
     with torch.no_grad():
         nl = torch.FloatTensor([[0.3]])
         e = g.denoise_fn(xb, nl)
-    out["big_64_512"] = {"x_seed": 300, "noise_level": nl, "eps_crop": e[:, :, 192:320, 192:320].clone(),
+    out["big_64_512"] = {"x_seed": 300, "noise_level": nl, "eps_crop": _golden.sample(e[:, :, 192:320, 192:320]),
                          "eps_mean": e.mean().clone(), "eps_std": e.std().clone(), "eps_absmax": e.abs().max().clone()}
     torch.save(out, os.path.join(HERE, "sr3_golden.pt"))
     for f in ("schedules.pt", "sr3_golden.pt"):
-        print(f, os.path.getsize(os.path.join(HERE, f)) // 1024, "KiB")
+        size = os.path.getsize(os.path.join(HERE, f))
+        print(f, size // 1024, "KiB")
+        assert size <= 1_000_000, f"{f} is over 1 MB"
 
 
 if __name__ == "__main__":
